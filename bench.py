@@ -233,6 +233,48 @@ def parity_report(got: np.ndarray, delivered: int, wl: Workload, world: int, seq
                     "include/swarmdb_b200.h 'stream digests'; " + how}
 
 
+DUMP_RECORDS = 32_768            # --dump-outputs: records sampled from the step's 4,194,304 (32 MB of payload as float32)
+DUMP_SEED = 2024
+
+
+def dump_outputs(shard, out_dir: Path, local_rank: int, width: int) -> dict:
+    """Write what the last receive delivered (still on the device after an SDB_RECV_ASYNC receive) as DIR/<name>.npy:
+    every agent's record count, the step's totals, and for a fixed seeded sample of the records (`index`, positions in
+    delivery order) each header field and the payload bytes (one row of `width` bytes per record, zero past its len).
+    float64 where the values are integers that float32 cannot hold exactly; float32 for counts and payload bytes."""
+    from cuda.bindings import runtime as cudart
+    from swarmdb_b200._native import HDR_DTYPE
+    total, pbytes = shard.last_receive_totals()
+    cnt_dev, hdr_dev, pay_dev = shard.last_receive_dev()
+    counts = np.empty(shard.stats()["n_agents"], np.uint32)
+    hdr = np.empty(total, HDR_DTYPE)
+    pay = np.empty(pbytes, np.uint8)
+    assert cudart.cudaSetDevice(local_rank)[0] == cudart.cudaError_t.cudaSuccess
+    for host, dev in ((counts, cnt_dev), (hdr, hdr_dev), (pay, pay_dev)):
+        err = cudart.cudaMemcpy(host.ctypes.data, dev, host.nbytes, cudart.cudaMemcpyKind.cudaMemcpyDeviceToHost)[0]
+        assert err == cudart.cudaError_t.cudaSuccess, err
+    assert int(counts.sum()) == total
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(total, min(total, DUMP_RECORDS), replace=False))
+    lens = hdr["len"].astype(np.int64)
+    start = np.concatenate(([0], np.cumsum((lens + 31) // 32 * 32)))[idx]        # payloads back to back, 32-byte padded
+    col = np.arange(width)
+    inside = col[None, :] < lens[idx][:, None]
+    rows = np.where(inside, pay[np.minimum(start[:, None] + col[None, :], pbytes - 1)], 0)
+    sample = hdr[idx]
+    assert int(hdr["seq"].max()) < 2 ** 53                                      # exact in float64
+    arrays = {"counts": counts.astype(np.float32), "totals": np.array([total, pbytes], np.float64),
+              "index": idx.astype(np.float64), "payload": rows.astype(np.float32)}
+    for f in HDR_DTYPE.names:
+        arrays[f"header_{f}"] = sample[f].astype(np.float64)
+    nbytes = sum(a.nbytes for a in arrays.values())
+    assert nbytes <= 64 << 20, nbytes
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+    return {"dir": str(out_dir), "files": sorted(f"{n}.npy" for n in arrays), "bytes": nbytes, "records": total,
+            "records_sampled": len(idx)}
+
+
 WORKLOAD_C2 = ("c2: 1M agents, 15625 groups x 64, 65536 group sends/step (4,194,304 routed msgs), "
                "256-byte payloads, full drain (receive_batch all agents, max_messages=100) each step")
 
@@ -272,7 +314,7 @@ def run_reference(args, rank, world):
     per, routed = [], 0
     t0 = time.perf_counter()
     k = 0
-    while k < max(args.steps, 1) and (time.perf_counter() - t0) < 150.0:
+    while k < args.steps:
         t1 = time.perf_counter()
         r, drained, _ = o.mt_group_roundtrip(cores, *batches[k % 2], max_messages=100)
         per.append((time.perf_counter() - t1) * 1e3)
@@ -519,6 +561,9 @@ def run_gpu(args, rank, world, local_rank):
         launches = st1["kernel_launches"] - launches0
         delivered = st1["delivered"] - st0["delivered"]          # counted on the device by the receive kernels
         assert st1["ring_overflow"] == 0 and shard.last_receive_totals()[0] == per_step_msgs
+        if args.dump_outputs:                              # untimed; before the sustained block reuses the receive buffers
+            info = dump_outputs(shard, Path(args.dump_outputs), local_rank, wl.L)
+            print(f"bench.py: step {W + K - 1} outputs written: {json.dumps(info)}", file=sys.stderr, flush=True)
         # sustained figure: the same step repeated for a few hundred milliseconds (clocks and power settle), timed as one block
         sustained = None
         if args.sustained_steps > 0:
@@ -729,10 +774,17 @@ def main():
     ap.add_argument("--sustained-steps", type=int, default=300,
                     help="extra block of steps after the K timed ones, timed as a whole and reported under `sustained` (0 = skip)")
     ap.add_argument("--no-extras", action="store_true", help="profiling runs: only the device-resident timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one delivered (per-agent counts, a seeded sample of "
+                         "the records' headers and payloads) as DIR/<name>.npy; one GPU only")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or world != 1):
+        ap.error("--dump-outputs needs the GPU arm on one GPU (--impl ours, no torchrun)")
     if args.warmup < 3:
         args.warmup = 3
     if args.no_extras:

@@ -15,17 +15,15 @@ from __future__ import annotations
 import hashlib
 import shutil
 import sys
-from pathlib import Path
 
-HERE = Path(__file__).resolve().parent
-REF_DIR = HERE / "_ref"
-STAGED = REF_DIR / "swarmdb_reference_main.py"
-SOURCE = Path("/root/reference/swarmdb/ main.py")
+from oracle.ref_loader import REFERENCE_MAIN as SOURCE, STAGED_MAIN as STAGED, readable_file
+
+REF_DIR = STAGED.parent
 
 
 def build(quiet: bool = False) -> bool:
     """Returns True when oracle/_ref holds the reference file (freshly staged or already there)."""
-    if not SOURCE.is_file():
+    if not readable_file(SOURCE):
         if not quiet:
             print(f"oracle/_ref: {SOURCE} not present here; keeping whatever is staged", file=sys.stderr)
         return STAGED.is_file()

@@ -34,11 +34,19 @@ STAGED_MAIN = Path(__file__).resolve().parent / "_ref" / "swarmdb_reference_main
 _STUB_DIR = Path(__file__).resolve().parent / "kafka_stub"
 
 
+def readable_file(path: Path) -> bool:
+    """True when `path` is a file this user can read; a directory it may not enter counts as absent."""
+    try:
+        return path.is_file() and os.access(path, os.R_OK)
+    except OSError:
+        return False
+
+
 def reference_path():
     """The unmodified reference file: in place when /root/reference exists, else the staged copy, else None."""
-    if REFERENCE_MAIN.is_file():
+    if readable_file(REFERENCE_MAIN):
         return REFERENCE_MAIN
-    if STAGED_MAIN.is_file():
+    if readable_file(STAGED_MAIN):
         return STAGED_MAIN
     return None
 
